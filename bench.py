@@ -3,7 +3,7 @@
 the ORB extractor on the left and right images -- on synthetic 1242x375 stereo frames (centre-cropped to the
 net's 1024x352 like System::TrackStereo does), N x B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--model basic|standard] [--T 6]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--model basic|standard] [--T 6] [--dump-outputs DIR]
 
 One "step" = one stereo frame through both operators.  `value` times the operators with the cropped inputs
 already resident in HBM; `e2e` times the reference-facing calls (segmentImage / operator()) on HOST buffers,
@@ -16,6 +16,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -27,13 +28,23 @@ sys.path.insert(0, os.path.join(ROOT, "tools"))
 
 CROP_X, CROP_Y, NET_W, NET_H = 109, 11, 1024, 352
 BASELINE_PUBLISHED = None  # BASELINE.md holds no published number for this metric
+DUMP_BYTES = 64 << 20  # --dump-outputs writes at most this much
+
+
+def count_arg(minimum):
+    def parse(text):
+        v = int(text)
+        if v < minimum:
+            raise argparse.ArgumentTypeError(f"must be at least {minimum}")
+        return v
+    return parse
 
 
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=30)
-    ap.add_argument("--warmup", type=int, default=5)
+    ap.add_argument("--steps", type=count_arg(1), default=30, help="timed steps")
+    ap.add_argument("--warmup", type=count_arg(0), default=5, help="untimed steps before them")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--model", default="basic", choices=["basic", "standard"])
     ap.add_argument("--T", type=int, default=0, help="MC samples (default 6 basic / 12 standard; 6 standard for N>1)")
@@ -45,7 +56,12 @@ def parse_args():
                     help="--impl reference: full frames per step if (warmup + steps) of them fit this budget, else bounded samples")
     ap.add_argument("--sustain-seconds", type=float, default=3.0,
                     help="extra sustained leg on rank 0 (N=1): frames back to back for this long, own clock samples (0 = skip)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (rank 0's frame) to DIR/<name>.npy; see dump_outputs")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return args
 
 
 def model_files(kind, T, cache_dir):
@@ -75,6 +91,28 @@ def frames(n, start=0):
         gr = np.ascontiguousarray(bgr_to_gray(right)[CROP_Y:CROP_Y + NET_H, CROP_X:CROP_X + NET_W])
         out.append((left, gl, gr))
     return out
+
+
+def dump_outputs(out_dir, rec, conf, ent):
+    """Writes one timed step's results as out_dir/<name>.npy, in float32 or float64, so that two builds can be compared output
+    for output: `classes`, `confidence` and `entropy` (SegNet's [H, W] maps, the latter two in double), `record_confidence` and
+    `record_entropy` (the single-precision copies written into the packed record), and per image (`_left`, `_right`)
+    `keypoints` [n, 7] (x, y, size, angle, response, octave, class_id) and `descriptors` [n, 32] (one byte per column).
+    `rec` is the step's unpacked record (sivo_b200/record.py).  Should the keypoints take the files past DUMP_BYTES, each image
+    keeps a fixed, seeded sample of its keypoint rows, in keypoint order."""
+    out = {"classes": rec["classes"].astype(np.float32), "confidence": conf, "entropy": ent,
+           "record_confidence": rec["confidence"].astype(np.float32), "record_entropy": rec["entropy"].astype(np.float32)}
+    max_rows = (DUMP_BYTES - sum(a.nbytes for a in out.values())) // (2 * 4 * (7 + 32))
+    for side in ("left", "right"):
+        kp, desc = rec["kp_" + side], rec["desc_" + side]
+        rows = np.arange(len(kp))
+        if len(rows) > max_rows:
+            rows = np.sort(np.random.default_rng(0).choice(len(kp), max_rows, replace=False))
+        out["keypoints_" + side] = np.stack([kp[f][rows].astype(np.float32) for f in kp.dtype.names], axis=1).reshape(-1, 7)
+        out["descriptors_" + side] = desc[rows].astype(np.float32)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class ClockSampler:
@@ -192,7 +230,8 @@ def run_reference(args, rank, world):
     import gen_prototxt
     from sivo_b200.prototxt import load_net
     T = args.T or (6 if args.model == "basic" else (12 if world == 1 else 6))  # the GPU arm's rule: configs[1] / [2] / [3]
-    net, proto, model, weights = model_files(args.model, T, os.path.join("/tmp", "sivo_b200_models"))
+    models = tempfile.TemporaryDirectory(prefix="sivo_b200_models_")
+    net, proto, model, weights = model_files(args.model, T, models.name)
     weights = weights or load_weights(net, model)
     cores = os.cpu_count() or 1
     fr = frames(1)
@@ -290,13 +329,10 @@ def main():
         os.environ.setdefault("NCCL_MAX_CTAS", nch)
         dist.init_process_group("nccl", device_id=dev)
     T = args.T or (6 if args.model == "basic" else (12 if world == 1 else 6))
-    cache = os.path.join("/tmp", "sivo_b200_models")
-    if rank == 0:
-        net, proto, model, weights = model_files(args.model, T, cache)
-    if world > 1:
-        dist.barrier()
-    if rank != 0:
-        net, proto, model, weights = model_files(args.model, T, cache)
+    # every rank writes its own copy of the seeded model into a directory of its own, removed at exit: nothing is shared
+    # with other runs or users, and the source tree may be read-only
+    models = tempfile.TemporaryDirectory(prefix="sivo_b200_models_")
+    net, proto, model, weights = model_files(args.model, T, models.name)
 
     seg = BayesianSegNet(BayesianSegNetParams(proto, model), device=local_rank, seed=1234, precision=args.precision,
                          engine=args.engine)
@@ -513,6 +549,10 @@ def main():
     gc.enable()
     if use_async_orb and (orb_l.device_status() or orb_r.device_status()):
         raise SystemExit("a pyramid level exceeded the device quad tree's capacity: the asynchronous records are not valid")
+    if args.dump_outputs and rank == 0:
+        # the last timed step's record and double maps, read before the legs below run device_step again
+        last = record.unpack(d_rec[(args.warmup + args.steps - 1) % NBUF].cpu().numpy(), NET_H, NET_W, kp_cap)
+        dump_outputs(args.dump_outputs, last, d_conf.cpu().numpy().reshape(NET_H, NET_W), d_ent.cpu().numpy().reshape(NET_H, NET_W))
     prof_value = dict(prof)  # the sustained leg and the e2e variants call device_step / the extractors again
     dev_ms = e0.elapsed_time(e1)
     elapsed = max(wall, dev_ms / 1e3)  # the ORB streams are the library's own; wall brackets everything (synced both sides)

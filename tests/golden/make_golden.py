@@ -1,9 +1,11 @@
-"""Regenerates the committed golden fixtures from the oracle (run in the build container; cv2 is used
-only to decode the PNG).  The fixtures let the -m gpu tests compare the CUDA path with known outputs
-even where cv2 / the oracle's dependencies differ, and pin the oracle against regressions.
+"""Regenerates the committed golden fixtures from the oracle (cv2 is used only to decode the PNG).  The
+fixtures let the -m gpu tests compare the CUDA path with known outputs even where cv2 / the oracle's
+dependencies differ, and pin the oracle against regressions.
 
   python tests/golden/make_golden.py
+  python tests/golden/make_golden.py --reference-topology <SIVO checkout>   # reference_topology.json only
 """
+import json
 import os
 import sys
 
@@ -28,7 +30,33 @@ def orb_record(gray, nfeatures):
                 cand_counts=np.array([len(c[0]) for c in r.candidates], np.int32))
 
 
+def layer_signature(net):
+    """What test_host.py compares of each layer: wiring, shapes and the sampling / normalisation parameters."""
+    return [[ly.name, ly.type, list(ly.bottoms), list(ly.tops), ly.num_output, ly.kernel, ly.pad, ly.local_size, ly.alpha,
+             ly.beta, ly.dropout_ratio, ly.sample_weights_test, ly.weight_filler] for ly in net.layers]
+
+
+REFERENCE_PROTOTXTS = {"basic": "config/bayesian_segnet/basic/kitti/bayesian_segnet_basic_kitti.prototxt",
+                       "standard": "config/bayesian_segnet/standard/kitti/bayesian_segnet_kitti.prototxt"}
+
+
+def reference_topology(ref_root):
+    """Layer signatures of the original SIVO project's two KITTI prototxts, one layer per line."""
+    from sivo_b200.prototxt import load_net
+    parts = []
+    for kind, rel in REFERENCE_PROTOTXTS.items():
+        net = load_net(open(os.path.join(ref_root, rel)).read())
+        layers = ",\n    ".join(json.dumps(s) for s in layer_signature(net))
+        parts.append(f'"{kind}": {{"source": {json.dumps(rel)}, "input_dims": {json.dumps(net.input_dims)}, "layers": [\n    {layers}]}}')
+    with open(os.path.join(HERE, "reference_topology.json"), "w") as f:
+        f.write("{" + ",\n".join(parts) + "}\n")
+
+
 def main():
+    if len(sys.argv) == 3 and sys.argv[1] == "--reference-topology":
+        reference_topology(sys.argv[2])
+        print("reference_topology.json written")
+        return
     img = cv2.imread(os.path.join(HERE, "kitti_000000_1242x375.png"))
     gray = np.ascontiguousarray(bgr_to_gray(img)[11:11 + 352, 109:109 + 1024])
     assert np.array_equal(bgr_to_gray(img), cv2.cvtColor(img, cv2.COLOR_BGR2GRAY))

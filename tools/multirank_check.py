@@ -5,6 +5,7 @@ rank's slice of the gathered buffer against its own recomputation of that rank's
 bit-identical maps; ORB is deterministic)."""
 import os
 import sys
+import tempfile
 
 import numpy as np
 
@@ -24,10 +25,8 @@ def main():
     dev = torch.device("cuda", local)
     dist.init_process_group("nccl", device_id=dev)
     T = 2
-    if rank == 0:
-        model_files("basic", T, "/tmp/sivo_b200_models")
-    dist.barrier()
-    net, proto, model, _ = model_files("basic", T, "/tmp/sivo_b200_models")
+    models = tempfile.TemporaryDirectory(prefix="sivo_b200_models_")  # this rank's own copy of the seeded model
+    net, proto, model, _ = model_files("basic", T, models.name)
     hw = NET_H * NET_W
     nfeat = 1000
 
