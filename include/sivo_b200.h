@@ -69,6 +69,16 @@ int sivo_segnet_create(const char* prototxt, const char* caffemodel, int device,
                        sivo_segnet_t** out);
 int sivo_segnet_create_ex(const char* prototxt, const char* caffemodel, const sivo_segnet_options* opt,
                           sivo_segnet_t** out);
+/* Sample shard (latency mode of SURVEY 8e): a handle that computes Monte-Carlo samples [first_sample, first_sample + n_samples)
+ * of T (opt->T, or the prototxt's first dim).  T keeps the reference's rule T >= 2; a shard may hold a single sample.  Its op
+ * list has batch n_samples after the first sampling Dropout, and its dropout keys use the global sample index, so the shards
+ * of [0, T) compute exactly the samples of one unsharded handle.  SIVO_EINVAL if first_sample < 0, n_samples < 1 or
+ * first_sample + n_samples > T; SIVO_EFORMAT if the logits are not the 16-channel layout the MC kernels need.  On a shard with
+ * n_samples < T, sivo_segnet_run / _run_device / _run_device_maps return SIVO_EINVAL (their mean would be over the wrong
+ * sample count); a shard [0, T) behaves exactly like a handle from sivo_segnet_create_ex. */
+int sivo_segnet_create_shard(const char* prototxt, const char* caffemodel, const sivo_segnet_options* opt,
+                             int first_sample, int n_samples, sivo_segnet_t** out);
+/* T is the total sample count, also for a shard. */
 int sivo_segnet_geometry(const sivo_segnet_t* h, int* width, int* height, int* T, int* n_classes);
 /* Dropout masks are keyed by (seed, frame, layer, sample, element); frame auto-increments per run. */
 int sivo_segnet_set_frame(sivo_segnet_t* h, uint64_t frame);
@@ -90,6 +100,19 @@ int sivo_segnet_set_record_outputs(sivo_segnet_t* h, uint8_t* classes_device, fl
  * reduction; the double maps stay the operator's outputs (bayesian_segnet.cpp:192-203, 262-276 compute in double). */
 int sivo_segnet_run_device_maps(sivo_segnet_t* h, const uint8_t* bgr_device, uint8_t* classes_device, double* confidence_device,
                                 double* entropy_device, float* confidence_f32_device, float* entropy_f32_device, void* stream);
+/* The whole op list with the final reduction replaced by the per-pixel sum, in double, over this handle's samples of the
+ * softmax probabilities: prob_sum_device[c * H*W + p], n_classes planes.  accumulate = 0 overwrites, 1 adds to what is
+ * there (in sample order, so shards run one after another into one buffer give the unsharded sums bit for bit).  No host
+ * synchronisation; advances the frame counter like sivo_segnet_run_device.  A NULL stream is the handle's own stream, so
+ * shards that share one buffer are ordered by passing them one stream (or by events). */
+int sivo_segnet_run_device_partial(sivo_segnet_t* h, const uint8_t* bgr_device, double* prob_sum_device, int accumulate,
+                                   void* stream);
+/* classes / confidence / entropy (+ optional f32 copies; any output may be NULL) from the summed probabilities of all T
+ * samples, with the arithmetic of the single-handle reduction: equal sums give bit-identical maps.  The maps become the
+ * handle's last result, the one sivo_segnet_semantic_keys reads.  Does not advance the frame counter. */
+int sivo_segnet_finalize_device(sivo_segnet_t* h, const double* prob_sum_device, uint8_t* classes_device,
+                                double* confidence_device, double* entropy_device, float* confidence_f32_device,
+                                float* entropy_f32_device, void* stream);
 /* Test hook: copies blob `name` (any top in the prototxt; needs keep_blobs) to `out` as float NCHW.
  * `*n`, `*c`, `*hh`, `*ww` receive its shape; `out` may be NULL to query the shape only. */
 int sivo_segnet_blob(sivo_segnet_t* h, const char* name, float* out, size_t cap, int* n, int* c, int* hh,
@@ -209,6 +232,11 @@ int sivo_dbg_lrn(int device, const float* in, int n, int c, int h, int w, int si
                  float k, float* out);
 int sivo_dbg_mc_reduce(int device, const float* logits, int T, int c, int h, int w, uint8_t* classes,
                        double* confidence, double* entropy);
+/* The two halves of sivo_dbg_mc_reduce: sums[c][h][w] (+)= the softmax probabilities of T samples of logits (accumulate = 1
+ * adds to the sums passed in), and the maps from sums of T_total samples. */
+int sivo_dbg_mc_partial(int device, const float* logits, int T, int c, int h, int w, int accumulate, double* sums);
+int sivo_dbg_mc_finalize(int device, const double* sums, int T_total, int c, int h, int w, uint8_t* classes,
+                         double* confidence, double* entropy);
 int sivo_dbg_dropout_mask(int device, uint64_t seed, uint64_t frame, int layer, int T, int c, int h, int w,
                           uint8_t* keep);
 

@@ -43,6 +43,19 @@ int sivo_segnet_create_ex(const char* prototxt, const char* caffemodel, const si
   });
 }
 
+int sivo_segnet_create_shard(const char* prototxt, const char* caffemodel, const sivo_segnet_options* opt, int first_sample,
+                             int n_samples, sivo_segnet_t** out) {
+  return guarded([&] {
+    if (!out) fail(SIVO_EINVAL, "null output handle");
+    *out = nullptr;
+    if (n_samples < 1) fail(SIVO_EINVAL, "sample shard: n_samples = %d (need at least 1)", n_samples);
+    sivo_segnet_options o{};
+    if (opt) o = *opt;
+    auto* impl = new SegNet(prototxt ? prototxt : "", caffemodel ? caffemodel : "", o, first_sample, n_samples);
+    *out = new sivo_segnet{impl};
+  });
+}
+
 int sivo_segnet_create(const char* prototxt, const char* caffemodel, int device, uint64_t seed, sivo_segnet_t** out) {
   sivo_segnet_options o{};
   o.device = device;
@@ -109,6 +122,22 @@ int sivo_segnet_run_device_maps(sivo_segnet_t* h, const uint8_t* bgr_device, uin
     if (!h || !bgr_device) fail(SIVO_EINVAL, "null handle or image");
     h->impl->run_device(bgr_device, classes_device, confidence_device, entropy_device, static_cast<cudaStream_t>(stream),
                         confidence_f32_device, entropy_f32_device);
+  });
+}
+
+int sivo_segnet_run_device_partial(sivo_segnet_t* h, const uint8_t* bgr_device, double* prob_sum_device, int accumulate, void* stream) {
+  return guarded([&] {
+    if (!h || !bgr_device) fail(SIVO_EINVAL, "null handle or image");
+    h->impl->run_device_partial(bgr_device, prob_sum_device, accumulate, static_cast<cudaStream_t>(stream));
+  });
+}
+
+int sivo_segnet_finalize_device(sivo_segnet_t* h, const double* prob_sum_device, uint8_t* classes_device, double* confidence_device,
+                                double* entropy_device, float* confidence_f32_device, float* entropy_f32_device, void* stream) {
+  return guarded([&] {
+    if (!h) fail(SIVO_EINVAL, "null handle");
+    h->impl->finalize_device(prob_sum_device, classes_device, confidence_device, entropy_device, confidence_f32_device, entropy_f32_device,
+                             static_cast<cudaStream_t>(stream));
   });
 }
 
@@ -467,6 +496,38 @@ int sivo_dbg_mc_reduce(int device, const float* logits, int T, int c, int h, int
     if (classes) SIVO_CUDA(cudaMemcpy(classes, bc.p, static_cast<size_t>(h) * w, cudaMemcpyDeviceToHost));
     if (confidence) SIVO_CUDA(cudaMemcpy(confidence, bf.p, static_cast<size_t>(h) * w * 8, cudaMemcpyDeviceToHost));
     if (entropy) SIVO_CUDA(cudaMemcpy(entropy, be.p, static_cast<size_t>(h) * w * 8, cudaMemcpyDeviceToHost));
+  });
+}
+
+int sivo_dbg_mc_partial(int device, const float* logits, int T, int c, int h, int w, int accumulate, double* sums) {
+  return guarded([&] {
+    if (!logits || !sums || T <= 0 || c <= 0 || c > 16) fail(SIVO_EINVAL, "mc_partial: bad arguments");
+    SIVO_CUDA(cudaSetDevice(device));
+    const size_t bytes = static_cast<size_t>(c) * h * w * sizeof(double);
+    DevBuf bl, bs(bytes);
+    TensorView vl = make_view(bl, T, c, h, w, 16, DType::F32);
+    upload_nchw(logits, vl);
+    if (accumulate) SIVO_CUDA(cudaMemcpy(bs.p, sums, bytes, cudaMemcpyHostToDevice));
+    launch_mc_partial(static_cast<const float*>(vl.p), T, c, 16, h * w, bs.as<double>(), accumulate, nullptr);
+    SIVO_CUDA(cudaDeviceSynchronize());
+    SIVO_CUDA(cudaMemcpy(sums, bs.p, bytes, cudaMemcpyDeviceToHost));
+  });
+}
+
+int sivo_dbg_mc_finalize(int device, const double* sums, int T_total, int c, int h, int w, uint8_t* classes, double* confidence,
+                         double* entropy) {
+  return guarded([&] {
+    if (!sums || T_total <= 0 || c <= 0 || c > 16) fail(SIVO_EINVAL, "mc_finalize: bad arguments");
+    SIVO_CUDA(cudaSetDevice(device));
+    const size_t hw = static_cast<size_t>(h) * w;
+    DevBuf bs(static_cast<size_t>(c) * hw * sizeof(double)), bc(hw), bf(hw * 8), be(hw * 8);
+    SIVO_CUDA(cudaMemcpy(bs.p, sums, bs.bytes, cudaMemcpyHostToDevice));
+    launch_mc_finalize(bs.as<double>(), T_total, c, static_cast<int>(hw), bc.as<uint8_t>(), bf.as<double>(), be.as<double>(), nullptr,
+                       nullptr, nullptr);
+    SIVO_CUDA(cudaDeviceSynchronize());
+    if (classes) SIVO_CUDA(cudaMemcpy(classes, bc.p, hw, cudaMemcpyDeviceToHost));
+    if (confidence) SIVO_CUDA(cudaMemcpy(confidence, bf.p, hw * 8, cudaMemcpyDeviceToHost));
+    if (entropy) SIVO_CUDA(cudaMemcpy(entropy, be.p, hw * 8, cudaMemcpyDeviceToHost));
   });
 }
 

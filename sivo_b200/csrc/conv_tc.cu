@@ -76,6 +76,7 @@ struct TcParams {
   uint64_t seed;
   const uint64_t* frame;
   int drop_layer;
+  int drop_sample0;        // global index of batch image 0 (sample shards): the keep bits use drop_sample0 + img
   float drop_scale;
   // max-unpool fused into the epilogue (decoder convs): the output tensor is 2H x 2W and every pixel's channel
   // lands in the 2x2 position its pooling mask names, zeros elsewhere (upsample_layer.cpp:74-103)
@@ -304,7 +305,7 @@ __device__ __forceinline__ void epilogue_row(const TcParams& p, const TcConsts& 
       tmem_ld32(trow + cc, v);
       const int c0 = n0 + cc;
       if (p.has_drop && inside && ((c0 & 127) == 0 || cc == 0))
-        dropout_bits128(p.seed, *p.frame, p.drop_layer, img, static_cast<uint32_t>(y * p.W + x), c0 >> 7, bits);
+        dropout_bits128(p.seed, *p.frame, p.drop_layer, p.drop_sample0 + img, static_cast<uint32_t>(y * p.W + x), c0 >> 7, bits);
       const int wsel = (c0 >> 5) & 3;  // selects, not a dynamically indexed (= local-memory) array
       const uint32_t keep = !p.has_drop ? 0xFFFFFFFFu : wsel == 0 ? bits[0] : wsel == 1 ? bits[1] : wsel == 2 ? bits[2] : bits[3];
       uint4 e[4];
@@ -1310,6 +1311,9 @@ std::shared_ptr<ConvTcPlan> conv_tc_plan(const Op& op, const TensorView& in, con
   const int K = op.k;
   const int KW = op.fold_kw ? 1 : K;
   const bool roll = (in.cs == 64 || op.fold_kw) && !op.split;
+  // the kernel variant (image pairs, rows per block and with them the paired-tap kernel) follows the planning batch; only the
+  // grid follows the real one
+  const int plan_n = op.plan_n > 0 ? op.plan_n : in.n;
   if (op.fold_kw) {
     // window-folded input: `in` is the zero-padded 8-channel image [N][H][W + 8][8] half (3 zero pixels left, 5 right);
     // "pixel" x of the operand is the 128-byte window of 8 pixels x 8 channels starting at padded pixel x, i.e. image
@@ -1327,7 +1331,7 @@ std::shared_ptr<ConvTcPlan> conv_tc_plan(const Op& op, const TensorView& in, con
     cuuint64_t strides[3] = {static_cast<cuuint64_t>(in.cs) * 2, static_cast<cuuint64_t>(in.w) * in.cs * 2,
                              static_cast<cuuint64_t>(in.h) * in.w * in.cs * 2};
     const char* pk2_env = std::getenv("SIVO_B200_TC_PK2");
-    plan->pk2 = !roll && !op.split && K == 3 && in.w <= 64 && in.n >= 2 && !(pk2_env && pk2_env[0] == '0');
+    plan->pk2 = !roll && !op.split && K == 3 && in.w <= 64 && plan_n >= 2 && !(pk2_env && pk2_env[0] == '0');
     cuuint32_t box[4] = {64, static_cast<cuuint32_t>(plan->pk2 ? 64 : 128 + K - 1), 1, 1};
     encode(&plan->map_a, in.p, 4, dims, strides, box);
   }
@@ -1367,7 +1371,7 @@ std::shared_ptr<ConvTcPlan> conv_tc_plan(const Op& op, const TensorView& in, con
   const int cout_tiles = p.out_f32 == 1 ? 1 : op.cout_p / n_tile;
   const int n_z = plan->pk2 ? ceil_div(in.n, 2) : in.n;  // PK2: an image pair per tile
   const int columns = p.strips * n_z * cout_tiles;
-  const int rows = tc_rows(K, roll, n_tile, columns, in.h);
+  const int rows = tc_rows(K, roll, n_tile, p.strips * (plan->pk2 ? ceil_div(plan_n, 2) : plan_n) * cout_tiles, in.h);
   const int total_pairs = ceil_div(in.h, rows);
   // row blocks per CTA: minimise (waves of 148 SMs) x (blocks per CTA + ~1 block of prologue / halo overhead)
   int ppc = 1;
@@ -1389,7 +1393,7 @@ std::shared_ptr<ConvTcPlan> conv_tc_plan(const Op& op, const TensorView& in, con
     std::copy(op.h_bn_shift.begin(), op.h_bn_shift.end(), plan->cst.bn_shift);
   }
   p.out = out.p;
-  p.has_drop = 0; p.seed = 0; p.frame = nullptr; p.drop_layer = 0; p.drop_scale = 2.f;
+  p.has_drop = 0; p.seed = 0; p.frame = nullptr; p.drop_layer = 0; p.drop_sample0 = 0; p.drop_scale = 2.f;
   p.unpool_mask = nullptr; p.mask_n = 1;
   p.dbg_noshift = 0;
   p.dbg_noepi = 0;
@@ -1454,11 +1458,12 @@ std::shared_ptr<ConvTcPlan> conv_tc_plan(const Op& op, const TensorView& in, con
   return plan;
 }
 
-void conv_tc_set_dropout(ConvTcPlan& plan, uint64_t seed, const uint64_t* frame_dev, int layer, float scale) {
+void conv_tc_set_dropout(ConvTcPlan& plan, uint64_t seed, const uint64_t* frame_dev, int layer, int sample0, float scale) {
   plan.p.has_drop = 1;
   plan.p.seed = seed;
   plan.p.frame = frame_dev;
   plan.p.drop_layer = layer;
+  plan.p.drop_sample0 = sample0;
   plan.p.drop_scale = scale;
 }
 

@@ -136,6 +136,7 @@ void SegNet::build(const NetSpec& net, const WeightMap& weights) {
   };
   int drop_idx = 0;
   bool saw_softmax = false;
+  bool sampled = false;  // past the first sampling Dropout: tensors hold this handle's n_ samples
   for (size_t li = 0; li < net.layers.size(); ++li) {
     const LayerSpec& ly = net.layers[li];
     if (saw_softmax) fail(SIVO_EFORMAT, "prototxt: layers after Softmax are not on the path");
@@ -159,6 +160,7 @@ void SegNet::build(const NetSpec& net, const WeightMap& weights) {
         op.in = in;
         op.k = ly.kernel; op.pad = ly.pad; op.cin = iv.c; op.cout = ly.num_output;
         op.cin_p = iv.cs;
+        if (sampled) op.plan_n = T_;  // a shard's per-sample layers run the unsharded handle's kernel variants
         const char* no_tc = std::getenv("SIVO_B200_NO_TC");
         if (iv.cs == 4 && iv.c == 3 && act_ == DType::F16 && opt_.engine != SIVO_ENGINE_SIMT && (ly.kernel == 7 || ly.kernel == 3) &&
             ly.num_output % 64 == 0 && !(no_tc && no_tc[0] == '1')) {
@@ -238,7 +240,7 @@ void SegNet::build(const NetSpec& net, const WeightMap& weights) {
         op.flops = 2.0 * iv.c * ly.kernel * ly.kernel * op.cout * iv.h * iv.w * iv.n;  // algorithmic, whatever the mapping
         op.flops_exec = op.split ? 3.0 * op.flops : op.flops;
         flops_dedup += op.flops;
-        flops_naive += op.flops / iv.n * T_;
+        flops_naive += op.flops / iv.n * n_;
         if (logits && !opt_.keep_blobs && op.k == 1 && op.cin == 64 && op.cout <= 16 && !op.relu && !bn && !ops_.empty() &&
             ops_.back().kind == Op::Conv && ops_.back().use_tc && ops_.back().out == in && conv_tc_can_fuse_classifier(*ops_.back().tc)) {
           // 1x1 classifier straight after a tensor-core convolution: computed in that convolution's epilogue from the
@@ -353,10 +355,10 @@ void SegNet::build(const NetSpec& net, const WeightMap& weights) {
         }
         if (ly.dropout_ratio != 0.5f)
           fail(SIVO_EFORMAT, "layer '%s': dropout_ratio %.3f (the keep-bit rule is specified for 0.5)", ly.name.c_str(), ly.dropout_ratio);
-        if (!ops_.empty() && ops_.back().kind == Op::Conv && ops_.back().use_tc && ops_.back().out == in && iv.n == T_ &&
+        if (sampled && !ops_.empty() && ops_.back().kind == Op::Conv && ops_.back().use_tc && ops_.back().out == in && iv.n == n_ &&
             iv.dt == DType::F16 && ly.tops[0] == ly.bottoms[0]) {
           // in-place sampling Dropout right after a tensor-core convolution: applied in its epilogue registers
-          conv_tc_set_dropout(*ops_.back().tc, opt_.seed, d_frame_.as<uint64_t>(), drop_idx++, 1.f / (1.f - ly.dropout_ratio));
+          conv_tc_set_dropout(*ops_.back().tc, opt_.seed, d_frame_.as<uint64_t>(), drop_idx++, s0_, 1.f / (1.f - ly.dropout_ratio));
           ops_.back().layer += "+" + ly.name;
           break;
         }
@@ -366,8 +368,9 @@ void SegNet::build(const NetSpec& net, const WeightMap& weights) {
         op.in = in;
         op.drop_layer = drop_idx++;
         op.drop_scale = 1.f / (1.f - ly.dropout_ratio);
-        op.out = add_tensor(ly.tops[0], T_, iv.c, iv.h, iv.w, iv.cs, act_);
+        op.out = add_tensor(ly.tops[0], n_, iv.c, iv.h, iv.w, iv.cs, act_);
         ops_.push_back(std::move(op));
+        sampled = true;
         break;
       }
       case LayerType::Softmax: {
@@ -384,9 +387,12 @@ void SegNet::build(const NetSpec& net, const WeightMap& weights) {
     }
   }
   if (!saw_softmax) fail(SIVO_EFORMAT, "prototxt: no Softmax output layer ('prob')");
+  if (!sampled && n_ != T_) fail(SIVO_EINVAL, "sample shard of a net without a sampling Dropout layer: every sample is the same");
 }
 
-SegNet::SegNet(const std::string& prototxt, const std::string& caffemodel, const sivo_segnet_options& opt) : opt_(opt) {
+SegNet::SegNet(const std::string& prototxt, const std::string& caffemodel, const sivo_segnet_options& opt, int first_sample,
+               int n_samples)
+    : opt_(opt) {
   // checkConfig (bayesian_segnet.cpp:80-89)
   if (prototxt.empty()) fail(SIVO_EINVAL, "model_file (.prototxt file) is empty!");
   if (caffemodel.empty()) fail(SIVO_EINVAL, "weights_file (.caffemodel file) is empty!");
@@ -395,6 +401,11 @@ SegNet::SegNet(const std::string& prototxt, const std::string& caffemodel, const
   // bayesian_segnet.cpp:65-70
   if (net.dims[1] != 3) fail(SIVO_EINVAL, "Input layer must have 3 channels!");
   if (T_ <= 1) fail(SIVO_EINVAL, "Input layer must have a batch size greater than 1!");
+  if (n_samples >= 0 && (first_sample < 0 || n_samples < 1 || first_sample > T_ - n_samples))
+    fail(SIVO_EINVAL, "sample shard [%d, %d + %d) is not a non-empty range inside the T = %d Monte-Carlo samples", first_sample,
+         first_sample, n_samples, T_);
+  s0_ = n_samples >= 0 ? first_sample : 0;
+  n_ = n_samples >= 0 ? n_samples : T_;
   H_ = net.dims[2];
   W_ = net.dims[3];
   if (H_ <= 0 || W_ <= 0) fail(SIVO_EFORMAT, "prototxt: bad input geometry %dx%d", W_, H_);
@@ -406,6 +417,11 @@ SegNet::SegNet(const std::string& prototxt, const std::string& caffemodel, const
   try {  // a malformed model throws out of build(): the destructor does not run for a half-built object
     d_frame_.alloc(sizeof(FrameArgs));
     build(net, weights);
+    if (n_samples >= 0) {  // the partial / finalize kernels read 16-float logit pixels
+      const TensorView& lv = tensors_[ops_.back().in]->v;
+      if (lv.cs != 16 || lv.c > 16)
+        fail(SIVO_EFORMAT, "sample shards need logits in the 16-channel layout (%d classes, channel stride %d)", lv.c, lv.cs);
+    }
   } catch (...) {
     cudaStreamDestroy(stream_);
     stream_ = nullptr;
@@ -483,6 +499,7 @@ void SegNet::enqueue(const uint8_t* bgr_dev, uint8_t* classes_dev, double* conf_
         d.seed = opt_.seed;
         d.frame_dev = d_frame_.as<uint64_t>();
         d.layer = op.drop_layer;
+        d.sample0 = s0_;
         launch_dropout(tensors_[op.in]->v, tensors_[op.out]->v, d, op.drop_scale, s);
         break;
       }
@@ -491,13 +508,18 @@ void SegNet::enqueue(const uint8_t* bgr_dev, uint8_t* classes_dev, double* conf_
         d.seed = opt_.seed;
         d.frame_dev = d_frame_.as<uint64_t>();
         d.layer = op.drop_layer;
+        d.sample0 = s0_;
         const Tensor& mt = *tensors_[op.in2];
-        launch_dropout_unpool(tensors_[op.in]->v, T_, mt.buf.as<uint8_t>(), mt.v.n, tensors_[op.out]->v, d, op.drop_scale, s);
+        launch_dropout_unpool(tensors_[op.in]->v, n_, mt.buf.as<uint8_t>(), mt.v.n, tensors_[op.out]->v, d, op.drop_scale, s);
         break;
       }
       case Op::Reduce: {
         if (skip_reduce_) break;
         const TensorView& lv = tensors_[op.in]->v;
+        if (partial_) {
+          launch_mc_partial(static_cast<const float*>(lv.p), lv.n, lv.c, lv.cs, lv.h * lv.w, nullptr, 0, s, d_frame_.as<FrameArgs>());
+          break;
+        }
         launch_mc_reduce(static_cast<const float*>(lv.p), lv.n, lv.c, lv.cs, lv.h * lv.w, classes_dev, conf_dev, ent_dev, s, 0, -1,
                          d_frame_.as<FrameArgs>());
         break;
@@ -545,17 +567,58 @@ void SegNet::semantic_keys(const sivo_keypoint* kps, int n, int max_static_class
   if (n_keep) *n_keep = kept;
 }
 
+void SegNet::require_whole(const char* what) const {
+  if (n_ != T_)
+    fail(SIVO_EINVAL, "%s: this handle computes Monte-Carlo samples [%d, %d) of T = %d only; run it with run_device_partial and "
+                      "finalize the summed probabilities", what, s0_, s0_ + n_, T_);
+}
+
 void SegNet::run_device(const uint8_t* bgr_dev, uint8_t* classes_dev, double* conf_dev, double* ent_dev, cudaStream_t s, float* conf32_dev,
                         float* ent32_dev) {
+  require_whole("run_device");
   SIVO_CUDA(cudaSetDevice(device_));
   if (!s) s = stream_;
   last_classes_ = classes_dev; last_conf_ = conf_dev; last_ent_ = ent_dev; last_stream_ = s;
+  FrameArgs fa{};
+  fa.bgr = bgr_dev; fa.classes = classes_dev; fa.conf = conf_dev; fa.ent = ent_dev; fa.conf32 = conf32_dev; fa.ent32 = ent32_dev;
+  run_frame(fa, s);
+}
+
+void SegNet::run_device_partial(const uint8_t* bgr_dev, double* prob_sum_dev, int accumulate, cudaStream_t s) {
+  if (!prob_sum_dev) fail(SIVO_EINVAL, "run_device_partial: null probability-sum buffer");
+  SIVO_CUDA(cudaSetDevice(device_));
+  if (!s) s = stream_;
+  FrameArgs fa{};
+  fa.bgr = bgr_dev; fa.prob_sum = prob_sum_dev; fa.accumulate = accumulate ? 1 : 0;
+  partial_ = true;
+  try {
+    run_frame(fa, s);
+  } catch (...) {
+    partial_ = false;
+    throw;
+  }
+  partial_ = false;
+}
+
+void SegNet::finalize_device(const double* prob_sum_dev, uint8_t* classes_dev, double* conf_dev, double* ent_dev, float* conf32_dev,
+                             float* ent32_dev, cudaStream_t s) {
+  if (!prob_sum_dev) fail(SIVO_EINVAL, "finalize_device: null probability-sum buffer");
+  SIVO_CUDA(cudaSetDevice(device_));
+  if (!s) s = stream_;
+  launch_mc_finalize(prob_sum_dev, T_, n_classes_, H_ * W_, classes_dev, conf_dev, ent_dev, conf32_dev, ent32_dev, s);
+  last_classes_ = classes_dev; last_conf_ = conf_dev; last_ent_ = ent_dev; last_stream_ = s;
+}
+
+void SegNet::run_frame(const FrameArgs& frame_args, cudaStream_t s) {
+  const uint8_t* bgr_dev = frame_args.bgr;
+  uint8_t* classes_dev = frame_args.classes;
+  double* conf_dev = frame_args.conf;
+  double* ent_dev = frame_args.ent;
   // Everything that changes per frame -- the dropout frame counter and the caller's pointers -- goes to the device by value,
   // outside the captured graph (pipelined callers may issue the next frame before this one has started), so one graph per
   // stream serves every pointer set a caller cycles through
-  FrameArgs fa;
+  FrameArgs fa = frame_args;
   fa.frame = frame_++;
-  fa.bgr = bgr_dev; fa.classes = classes_dev; fa.conf = conf_dev; fa.ent = ent_dev; fa.conf32 = conf32_dev; fa.ent32 = ent32_dev;
   launch_set_frame_args(d_frame_.as<FrameArgs>(), fa, s);
   if (profiling_) {
     while (events_.size() < ops_.size() + 1) {
@@ -586,7 +649,7 @@ void SegNet::run_device(const uint8_t* bgr_dev, uint8_t* classes_dev, double* co
   if (graphs_enabled && graph_ok_ && all_tc) {
     // the graph's kernels read the image / result pointers from FrameArgs: the key is the stream (and the op-list variant) only
     const void* key[5] = {nullptr, nullptr, nullptr, nullptr,
-                          reinterpret_cast<const void*>(reinterpret_cast<uintptr_t>(s) ^ (skip_reduce_ ? 1u : 0u))};
+                          reinterpret_cast<const void*>(reinterpret_cast<uintptr_t>(s) ^ (skip_reduce_ ? 1u : 0u) ^ (partial_ ? 2u : 0u))};
     cudaGraphExec_t graph_exec_ = nullptr;
     for (size_t i = 0; i < graphs_.size(); ++i)
       if (memcmp(key, graphs_[i].key, sizeof key) == 0) {
@@ -634,6 +697,7 @@ void SegNet::run_device(const uint8_t* bgr_dev, uint8_t* classes_dev, double* co
 }
 
 void SegNet::run_host(const uint8_t* bgr, int rows, int cols, size_t stride, uint8_t* classes, double* conf, double* ent) {
+  require_whole("segmentImage");
   if (!bgr) fail(SIVO_EINVAL, "segmentImage: null image");
   // resizeImage (bayesian_segnet.cpp:142-162): exact size passes through, larger is centre-cropped;
   // smaller yields an empty Mat in the reference (and a crash downstream) -- here an error.

@@ -49,6 +49,9 @@ struct Op {
   DevBuf a_split;
   std::shared_ptr<ConvTcPlan> tc;
   bool use_tc = false;
+  // batch the tensor-core plan picks its kernel variant for (0: the input's own).  A sample shard plans its per-sample layers
+  // for all T samples, so that each sample's accumulation order -- and hence its logits -- is the unsharded handle's
+  int plan_n = 0;
   double flops = 0;       // algorithmic (the reference's operation count), for this op's batch
   double flops_exec = 0;  // what the launch executes: differs for the composed classifier (0.25x) and the split-operand mode (3x)
   // Dropout
@@ -58,11 +61,16 @@ struct Op {
 
 class SegNet {
  public:
-  SegNet(const std::string& prototxt, const std::string& caffemodel, const sivo_segnet_options& opt);
+  // n_samples < 0: all T samples.  Otherwise the handle computes samples [first_sample, first_sample + n_samples) of T (a
+  // sample shard): the op list after the first sampling Dropout has batch n_samples, and its dropout keys use the global index
+  SegNet(const std::string& prototxt, const std::string& caffemodel, const sivo_segnet_options& opt, int first_sample = 0,
+         int n_samples = -1);
   ~SegNet();
   int width() const { return W_; }
   int height() const { return H_; }
   int T() const { return T_; }
+  int first_sample() const { return s0_; }
+  int n_samples() const { return n_; }
   int classes() const { return n_classes_; }
   void set_frame(uint64_t f) { frame_ = f; }
   void run_host(const uint8_t* bgr, int rows, int cols, size_t stride, uint8_t* classes, double* conf, double* ent);
@@ -74,6 +82,12 @@ class SegNet {
   // conf32 / ent32 (optional): single-precision copies of the two maps, e.g. straight into the packed multi-GPU record
   void run_device(const uint8_t* bgr_dev, uint8_t* classes_dev, double* conf_dev, double* ent_dev, cudaStream_t s, float* conf32_dev = nullptr,
                   float* ent32_dev = nullptr);
+  // sample shards: the op list with the MC reduction replaced by the per-pixel double sums of this handle's softmax
+  // probabilities, prob_sum[c * H*W + p] (accumulate: add to what is there); advances the frame counter like run_device
+  void run_device_partial(const uint8_t* bgr_dev, double* prob_sum_dev, int accumulate, cudaStream_t s);
+  // the maps from the summed probabilities of all T samples; they become the last result (semantic_keys)
+  void finalize_device(const double* prob_sum_dev, uint8_t* classes_dev, double* conf_dev, double* ent_dev, float* conf32_dev,
+                       float* ent32_dev, cudaStream_t s);
   void semantic_keys(const sivo_keypoint* kps, int n, int max_static_class, uint8_t* kp_class, double* kp_conf, double* kp_entropy,
                      int* keep_idx, int* n_keep);
   void blob(const std::string& name, float* out, size_t cap, int* n, int* c, int* h, int* w);
@@ -90,9 +104,12 @@ class SegNet {
   void build(const NetSpec& net, const WeightMap& weights);
   void prepare_conv(Op& op, const std::vector<Blob>& conv_blobs, const std::vector<Blob>* bn_blobs);
   void enqueue(const uint8_t* bgr_dev, uint8_t* classes_dev, double* conf_dev, double* ent_dev, cudaStream_t s, bool timed);
+  void run_frame(const FrameArgs& fa, cudaStream_t s);
+  void require_whole(const char* what) const;  // refuses whole-frame calls on a shard that holds only part of the T samples
 
   sivo_segnet_options opt_;
   int device_ = 0, T_ = 0, H_ = 0, W_ = 0, n_classes_ = 0;
+  int s0_ = 0, n_ = 0;  // this handle's samples [s0_, s0_ + n_) of T_ (n_ == T_ unless it is a sample shard)
   DType act_ = DType::F16;
   uint64_t frame_ = 0;
   bool profiling_ = false;
@@ -120,6 +137,7 @@ class SegNet {
   // segmentImage read-back overlap: the MC reduction runs in row bands and each band's slices of the three maps start their
   // device-to-host copy on a second stream while the next band is reduced
   bool skip_reduce_ = false;      // set by run_host around run_device: the op list stops before the Reduce op
+  bool partial_ = false;          // set by run_device_partial: the Reduce op writes the probability sums (FrameArgs::prob_sum)
   cudaStream_t copy_stream_ = nullptr;
   std::vector<cudaEvent_t> band_ev_;
   // device-resident copies run_host leaves for a packed multi-GPU record (set_record_outputs)
@@ -132,8 +150,8 @@ class SegNet {
 bool conv_tc_supported(const Op& op, const TensorView& in, const TensorView& out);
 std::shared_ptr<ConvTcPlan> conv_tc_plan(const Op& op, const TensorView& in, const TensorView& out, const void* w_tc);
 void conv_tc_launch(const ConvTcPlan& plan, const Op& op, cudaStream_t s);
-// fuses the sampling Dropout that follows the convolution in place into its epilogue
-void conv_tc_set_dropout(ConvTcPlan& plan, uint64_t seed, const uint64_t* frame_dev, int layer, float scale);
+// fuses the sampling Dropout that follows the convolution in place into its epilogue; batch image i is sample sample0 + i
+void conv_tc_set_dropout(ConvTcPlan& plan, uint64_t seed, const uint64_t* frame_dev, int layer, int sample0, float scale);
 // fuses the max-unpool (Upsample) that consumes the convolution's output into its epilogue; `out_2h_2w` is the
 // unpooled tensor the convolution then writes instead of its own output
 void conv_tc_set_unpool(ConvTcPlan& plan, const uint8_t* mask, int mask_n, void* out_2h_2w);

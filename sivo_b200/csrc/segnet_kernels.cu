@@ -192,7 +192,7 @@ __global__ void k_unpool(const AT* __restrict__ in, const uint8_t* __restrict__ 
 // ---- test-time dropout sampling (dropout_layer.cpp:31-46): y = x * keep * 1/(1-ratio).
 template <typename AT>
 __global__ void k_dropout(const AT* __restrict__ in, int in_n, AT* __restrict__ out, int N, int HW, int cs, int C,
-                          uint64_t seed, const uint64_t* __restrict__ frame, int layer, float scale) {
+                          uint64_t seed, const uint64_t* __restrict__ frame, int layer, int sample0, float scale) {
   size_t i = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;  // one thread per (n, pix, 32-ch word)
   int words = (cs + 31) / 32;
   size_t total = static_cast<size_t>(N) * HW * words;
@@ -202,7 +202,7 @@ __global__ void k_dropout(const AT* __restrict__ in, int in_n, AT* __restrict__ 
   uint32_t pix = r % HW;
   int n = r / HW;
   uint32_t bits[4];
-  dropout_bits128(seed, *frame, layer, n, pix, wd >> 2, bits);
+  dropout_bits128(seed, *frame, layer, sample0 + n, pix, wd >> 2, bits);
   uint32_t b = bits[wd & 3];
   const AT* s = in + (static_cast<size_t>(n % in_n) * HW + pix) * cs + wd * 32;
   AT* d = out + (static_cast<size_t>(n) * HW + pix) * cs + wd * 32;
@@ -218,7 +218,7 @@ __global__ void k_dropout(const AT* __restrict__ in, int in_n, AT* __restrict__ 
 // is scattered straight into the 2x2 block its pooling mask names (dropout -> upsample pair of the decoder entry).
 template <bool UNPOOL>
 __global__ void k_dropout_h8(const uint4* __restrict__ in, int in_n, uint4* __restrict__ out, int N, int Hi, int Wi, int cs,
-                             uint64_t seed, const uint64_t* __restrict__ frame, int layer, float scale,
+                             uint64_t seed, const uint64_t* __restrict__ frame, int layer, int sample0, float scale,
                              const uint8_t* __restrict__ mask, int mask_n) {
   const size_t i = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
   const int chunks = cs >> 3;
@@ -229,7 +229,7 @@ __global__ void k_dropout_h8(const uint4* __restrict__ in, int in_n, uint4* __re
   const uint32_t pix = static_cast<uint32_t>(r % HW);
   const int n = static_cast<int>(r / HW);
   uint32_t bits[4];
-  dropout_bits128(seed, *frame, layer, n, pix, ch >> 4, bits);
+  dropout_bits128(seed, *frame, layer, sample0 + n, pix, ch >> 4, bits);
   const uint32_t b = (bits[(ch >> 2) & 3] >> ((ch & 3) * 8)) & 0xFFu;
   const uint4 v = __ldg(in + (static_cast<size_t>(n % in_n) * HW + pix) * chunks + ch);
   const uint32_t w[4] = {v.x, v.y, v.z, v.w};
@@ -329,20 +329,15 @@ __global__ void k_mc_reduce(const float* __restrict__ logits, int T, int cs, int
 // Same reduction with four lanes per pixel (one float4 = 4 classes each): a warp reads 512 contiguous bytes per
 // sample and there are 4x more threads in flight, which is what this HBM-bound pass needs.  The softmax max / sum and
 // the final argmax / entropy are combined with xor-shuffles inside the 4-lane group (first maximum still wins).
-__global__ void k_mc_reduce_quad(const float* __restrict__ logits, int T, int C, int hw, uint8_t* __restrict__ classes,
-                                 double* __restrict__ conf, double* __restrict__ entropy, int pix0, int pix_end,
-                                 const FrameArgs* __restrict__ args) {
-  float *conf32 = nullptr, *ent32 = nullptr;
-  if (args) { classes = args->classes; conf = args->conf; entropy = args->ent; conf32 = args->conf32; ent32 = args->ent32; }
-  // Instruction diet (ncu: the first version was issue-bound at 3400 instructions per warp, 0.8 TB/s): one IEEE
-  // reciprocal per sample instead of C divisions (p = e * (1/sum), <= 1 ulp from e/sum), mean = acc * (1/T) in double,
-  // and log2 evaluated in float on the double mean (relative error < 2^-22, i.e. < 1e-6 on the entropy, against the
-  // 1e-4 the contract allows); the products and the sums stay in double like computeEntropy (bayesian_segnet.cpp:38-44).
-  const int gid = blockIdx.x * blockDim.x + threadIdx.x;
-  const int pix = pix0 + (gid >> 2), q = gid & 3;
-  const bool live = pix < pix_end;
-  const int pp = live ? pix : hw - 1;
-  double acc[4] = {0.0, 0.0, 0.0, 0.0};
+// Instruction diet (ncu: the first version was issue-bound at 3400 instructions per warp, 0.8 TB/s): one IEEE
+// reciprocal per sample instead of C divisions (p = e * (1/sum), <= 1 ulp from e/sum), mean = acc * (1/T) in double,
+// and log2 evaluated in float on the double mean (relative error < 2^-22, i.e. < 1e-6 on the entropy, against the
+// 1e-4 the contract allows); the products and the sums stay in double like computeEntropy (bayesian_segnet.cpp:38-44).
+// The two halves -- per-sample softmax summed into acc, then mean / argmax / entropy -- are shared by the one-pass
+// reduction and the partial / finalize pair of sample shards, so equal sums give bit-identical maps.
+
+// lane q of pixel pp: acc[j] += softmax probability of class 4q + j, for samples 0..T-1 of `logits`, in sample order
+__device__ __forceinline__ void mc_quad_accumulate(const float* __restrict__ logits, int T, int C, int hw, int pp, int q, double acc[4]) {
   constexpr int kBatch = 6;  // samples whose loads are issued together (memory-level parallelism: the pass is HBM-bound)
   for (int t0 = 0; t0 < T; t0 += kBatch) {
   float4 vb[kBatch];
@@ -372,9 +367,14 @@ __global__ void k_mc_reduce_quad(const float* __restrict__ logits, int T, int C,
     for (int j = 0; j < 4; ++j) acc[j] += static_cast<double>(__fmul_rn(x[j], inv));
   }
   }
+}
+
+// mean over T, first-max argmax and entropy from the 4-lane group's sums; every lane of the group ends with the pixel's result
+__device__ __forceinline__ void mc_quad_finalize(const double acc[4], int T, int C, int q, double& best, int& arg, double& ent) {
   const double inv_t = 1.0 / static_cast<double>(T);
-  double best = -1.0, ent = 0.0;
-  int arg = 0;
+  best = -1.0;
+  ent = 0.0;
+  arg = 0;
 #pragma unroll
   for (int j = 0; j < 4; ++j) {
     if (q * 4 + j >= C) continue;
@@ -390,6 +390,68 @@ __global__ void k_mc_reduce_quad(const float* __restrict__ logits, int T, int C,
     ent += __shfl_xor_sync(0xffffffffu, ent, o);
     if (ob > best || (ob == best && oa < arg)) { best = ob; arg = oa; }
   }
+}
+
+__global__ void k_mc_reduce_quad(const float* __restrict__ logits, int T, int C, int hw, uint8_t* __restrict__ classes,
+                                 double* __restrict__ conf, double* __restrict__ entropy, int pix0, int pix_end,
+                                 const FrameArgs* __restrict__ args) {
+  float *conf32 = nullptr, *ent32 = nullptr;
+  if (args) { classes = args->classes; conf = args->conf; entropy = args->ent; conf32 = args->conf32; ent32 = args->ent32; }
+  const int gid = blockIdx.x * blockDim.x + threadIdx.x;
+  const int pix = pix0 + (gid >> 2), q = gid & 3;
+  const bool live = pix < pix_end;
+  const int pp = live ? pix : hw - 1;
+  double acc[4] = {0.0, 0.0, 0.0, 0.0};
+  mc_quad_accumulate(logits, T, C, hw, pp, q, acc);
+  double best, ent;
+  int arg;
+  mc_quad_finalize(acc, T, C, q, best, arg, ent);
+  if (live && q == 0) {
+    if (classes) classes[pix] = static_cast<uint8_t>(arg);
+    if (conf) conf[pix] = best;
+    if (entropy) entropy[pix] = ent;
+    if (conf32) conf32[pix] = static_cast<float>(best);
+    if (ent32) ent32[pix] = static_cast<float>(ent);
+  }
+}
+
+// Sample shards, first half: the same 4-lane softmax, continued from the sums already in prob_sum ([C][hw] doubles) or from 0.
+// Adding the shards of [0, T) one after another in sample order performs exactly k_mc_reduce_quad's sequence of double additions.
+__global__ void k_mc_partial_quad(const float* __restrict__ logits, int n, int C, int hw, double* __restrict__ prob_sum, int accumulate,
+                                  const FrameArgs* __restrict__ args) {
+  if (args) { prob_sum = args->prob_sum; accumulate = args->accumulate; }
+  const int gid = blockIdx.x * blockDim.x + threadIdx.x;
+  const int pix = gid >> 2, q = gid & 3;
+  const bool live = pix < hw;
+  const int pp = live ? pix : hw - 1;
+  double acc[4] = {0.0, 0.0, 0.0, 0.0};
+  if (accumulate && live) {
+#pragma unroll
+    for (int j = 0; j < 4; ++j)
+      if (q * 4 + j < C) acc[j] = prob_sum[static_cast<size_t>(q * 4 + j) * hw + pix];
+  }
+  mc_quad_accumulate(logits, n, C, hw, pp, q, acc);
+  if (!live) return;
+#pragma unroll
+  for (int j = 0; j < 4; ++j)
+    if (q * 4 + j < C) prob_sum[static_cast<size_t>(q * 4 + j) * hw + pix] = acc[j];
+}
+
+// Second half: the maps from the summed probabilities of all T samples (the tail of k_mc_reduce_quad)
+__global__ void k_mc_finalize(const double* __restrict__ prob_sum, int T, int C, int hw, uint8_t* __restrict__ classes,
+                              double* __restrict__ conf, double* __restrict__ entropy, float* __restrict__ conf32,
+                              float* __restrict__ ent32) {
+  const int gid = blockIdx.x * blockDim.x + threadIdx.x;
+  const int pix = gid >> 2, q = gid & 3;
+  const bool live = pix < hw;
+  const int pp = live ? pix : hw - 1;
+  double acc[4] = {0.0, 0.0, 0.0, 0.0};
+#pragma unroll
+  for (int j = 0; j < 4; ++j)
+    if (q * 4 + j < C) acc[j] = prob_sum[static_cast<size_t>(q * 4 + j) * hw + pp];
+  double best, ent;
+  int arg;
+  mc_quad_finalize(acc, T, C, q, best, arg, ent);
   if (live && q == 0) {
     if (classes) classes[pix] = static_cast<uint8_t>(arg);
     if (conf) conf[pix] = best;
@@ -717,7 +779,7 @@ void launch_dropout(TensorView in, TensorView out, const DropoutParams& d, float
   if (in.dt == DType::F16 && out.dt == DType::F16 && out.cs % 8 == 0 && out.c == out.cs && in.cs == out.cs) {
     const size_t total = static_cast<size_t>(out.n) * out.h * out.w * (out.cs / 8);
     k_dropout_h8<false><<<blocks_for(total, 256), 256, 0, s>>>(static_cast<const uint4*>(in.p), in.n, static_cast<uint4*>(out.p), out.n,
-                                                            out.h, out.w, out.cs, d.seed, d.frame_dev, d.layer, scale, nullptr, 1);
+                                                            out.h, out.w, out.cs, d.seed, d.frame_dev, d.layer, d.sample0, scale, nullptr, 1);
     SIVO_CUDA(cudaGetLastError());
     return;
   }
@@ -725,7 +787,7 @@ void launch_dropout(TensorView in, TensorView out, const DropoutParams& d, float
   size_t total = static_cast<size_t>(out.n) * out.h * out.w * words;
   DISPATCH_AT(in.dt, (k_dropout<AT><<<blocks_for(total, 256), 256, 0, s>>>(static_cast<const AT*>(in.p), in.n,
                                                                            static_cast<AT*>(out.p), out.n, out.h * out.w,
-                                                                           out.cs, out.c, d.seed, d.frame_dev, d.layer, scale)));
+                                                                           out.cs, out.c, d.seed, d.frame_dev, d.layer, d.sample0, scale)));
   SIVO_CUDA(cudaGetLastError());
 }
 
@@ -736,7 +798,7 @@ void launch_dropout_unpool(TensorView in, int T, const uint8_t* mask, int mask_n
     fail(SIVO_EINVAL, "dropout+unpool: unexpected tensor layout");
   const size_t total = static_cast<size_t>(T) * in.h * in.w * (in.cs / 8);
   k_dropout_h8<true><<<blocks_for(total, 256), 256, 0, s>>>(static_cast<const uint4*>(in.p), in.n, static_cast<uint4*>(out.p), T, in.h, in.w,
-                                                         in.cs, d.seed, d.frame_dev, d.layer, scale, mask, mask_n);
+                                                         in.cs, d.seed, d.frame_dev, d.layer, d.sample0, scale, mask, mask_n);
   SIVO_CUDA(cudaGetLastError());
 }
 
@@ -753,6 +815,22 @@ void launch_mc_reduce(const float* logits, int T, int C, int cs, int hw, uint8_t
   if (pix0 != 0 || npix != hw) fail(SIVO_EINVAL, "mc_reduce: pixel ranges need the 16-channel logits layout");
   if (C == 15) k_mc_reduce<15><<<blocks_for(hw, 128), 128, 0, s>>>(logits, T, cs, hw, classes, conf, entropy, args);
   else k_mc_reduce_generic<<<blocks_for(hw, 128), 128, 0, s>>>(logits, T, C, cs, hw, classes, conf, entropy, args);
+  SIVO_CUDA(cudaGetLastError());
+}
+
+void launch_mc_partial(const float* logits, int n, int C, int cs, int hw, double* prob_sum, int accumulate, cudaStream_t s,
+                       const FrameArgs* args) {
+  if (cs != 16 || C > 16) fail(SIVO_EFORMAT, "mc_partial: needs the 16-channel logits layout (%d classes, stride %d)", C, cs);
+  if (hw <= 0 || n <= 0) return;
+  k_mc_partial_quad<<<blocks_for(static_cast<size_t>(hw) * 4, 256), 256, 0, s>>>(logits, n, C, hw, prob_sum, accumulate, args);
+  SIVO_CUDA(cudaGetLastError());
+}
+
+void launch_mc_finalize(const double* prob_sum, int T, int C, int hw, uint8_t* classes, double* conf, double* entropy, float* conf32,
+                        float* ent32, cudaStream_t s) {
+  if (C > 16 || C <= 0 || T <= 0) fail(SIVO_EINVAL, "mc_finalize: %d classes, T = %d", C, T);
+  if (hw <= 0) return;
+  k_mc_finalize<<<blocks_for(static_cast<size_t>(hw) * 4, 256), 256, 0, s>>>(prob_sum, T, C, hw, classes, conf, entropy, conf32, ent32);
   SIVO_CUDA(cudaGetLastError());
 }
 

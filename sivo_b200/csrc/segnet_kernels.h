@@ -41,12 +41,15 @@ struct FrameArgs {
   double* ent;
   float* conf32;         // optional single-precision copies of the two maps (the packed multi-GPU record carries those)
   float* ent32;
+  double* prob_sum;      // partial runs (sample shards): [C][H*W] per-pixel sums of this handle's softmax probabilities
+  int accumulate;        // 0: the partial run overwrites prob_sum, 1: adds to it
 };
 
 struct DropoutParams {
   uint64_t seed = 0;
   const uint64_t* frame_dev = nullptr;  // device scalar, so a captured graph replays with a new frame
   int layer = 0;
+  int sample0 = 0;  // global index of the handle's first Monte-Carlo sample (sample shards); the keep bits use sample0 + n
 };
 
 // `args` != nullptr: the image / result pointers are read from *args on the device instead of the by-value arguments
@@ -78,6 +81,14 @@ void launch_dropout(TensorView in, TensorView out, const DropoutParams& d, float
 // pix0 / npix restrict the pass to pixels [pix0, pix0 + npix) (npix < 0: all of them)
 void launch_mc_reduce(const float* logits, int T, int C, int cs, int hw, uint8_t* classes, double* conf,
                       double* entropy, cudaStream_t s, int pix0 = 0, int npix = -1, const FrameArgs* args = nullptr);
+// The reduction split in two for sample shards.  partial: prob_sum[c * hw + p] (+)= sum over the n samples of `logits` (float
+// [n, H, W, 16]) of the softmax probabilities, in double and in sample order (accumulate = 0 starts from 0).  finalize: the
+// three maps (and optional f32 copies) from the sums of all T samples.  Partial over [0, T) + finalize is bitwise
+// launch_mc_reduce.  `args` != nullptr: prob_sum / accumulate (partial) or the map pointers (finalize) come from *args.
+void launch_mc_partial(const float* logits, int n, int C, int cs, int hw, double* prob_sum, int accumulate, cudaStream_t s,
+                       const FrameArgs* args = nullptr);
+void launch_mc_finalize(const double* prob_sum, int T, int C, int hw, uint8_t* classes, double* conf, double* entropy, float* conf32,
+                        float* ent32, cudaStream_t s);
 void launch_dropout_bits(uint64_t seed, const uint64_t* frame_dev, int layer, int T, int C, int H, int W,
                          uint8_t* keep_nchw, cudaStream_t s);
 // layout converters for the test hooks (float NCHW host order <-> NHWC activation)

@@ -22,20 +22,29 @@ class BayesianSegNetParams:
 
 class BayesianSegNet:
     def __init__(self, params: BayesianSegNetParams, device: int = 0, seed: int = 1234, T: int = 0,
-                 precision: str = "fp16", engine: str = "auto", keep_blobs: bool = False):
+                 precision: str = "fp16", engine: str = "auto", keep_blobs: bool = False, samples: Optional[tuple] = None):
+        """samples = (first, count): a sample shard that computes Monte-Carlo samples [first, first + count) of T with the
+        dropout masks an unsharded handle draws for them (run_device_partial / finalize_device; segmentImage and run_device
+        refuse unless the shard covers all T samples)."""
         self._h = C.c_void_p()
         opt = L.SegnetOptions(device=device, T=T, seed=seed,
                               precision={"fp16": L.PRECISION_FP16, "fp32": L.PRECISION_FP32}[precision],
                               engine={"auto": L.ENGINE_AUTO, "simt": L.ENGINE_SIMT, "tcgen05": L.ENGINE_TCGEN05}[engine],
                               keep_blobs=int(keep_blobs), reserved=0)
-        rc = L.lib().sivo_segnet_create_ex(params.model_file.encode(), params.weights_file.encode(), C.byref(opt),
-                                           C.byref(self._h))
+        if samples is None:
+            rc = L.lib().sivo_segnet_create_ex(params.model_file.encode(), params.weights_file.encode(), C.byref(opt),
+                                               C.byref(self._h))
+        else:
+            first, count = (int(v) for v in samples)
+            rc = L.lib().sivo_segnet_create_shard(params.model_file.encode(), params.weights_file.encode(), C.byref(opt),
+                                                  first, count, C.byref(self._h))
         if rc == L.EINVAL:  # the reference throws std::invalid_argument (bayesian_segnet.cpp:66,68,82,86)
             raise ValueError(L.lib().sivo_last_error().decode())
         L.check(rc)
         w, h, t, nc = C.c_int(), C.c_int(), C.c_int(), C.c_int()
         L.check(L.lib().sivo_segnet_geometry(self._h, C.byref(w), C.byref(h), C.byref(t), C.byref(nc)))
         self.width, self.height, self.T, self.n_classes = w.value, h.value, t.value, nc.value
+        self.samples = (0, self.T) if samples is None else (first, count)
 
     def __del__(self):
         if getattr(self, "_h", None) and self._h.value and L is not None and getattr(L, "lib", None):
@@ -115,6 +124,20 @@ class BayesianSegNet:
         """run_device plus single-precision copies of the two maps (the packed multi-GPU record's layout); any pointer may be 0."""
         L.check(L.lib().sivo_segnet_run_device_maps(self._h, C.c_void_p(bgr_ptr), C.c_void_p(classes_ptr), C.c_void_p(conf_ptr),
                                                     C.c_void_p(ent_ptr), C.c_void_p(conf32_ptr), C.c_void_p(ent32_ptr), C.c_void_p(stream)))
+
+    def run_device_partial(self, bgr_ptr: int, sum_ptr: int, accumulate: bool = False, stream: int = 0):
+        """This handle's samples of one frame: sum_ptr (n_classes x H*W doubles) receives (accumulate: gains) the per-pixel
+        sums of their softmax probabilities.  Advances the frame counter."""
+        L.check(L.lib().sivo_segnet_run_device_partial(self._h, C.c_void_p(bgr_ptr), C.c_void_p(sum_ptr), int(bool(accumulate)),
+                                                       C.c_void_p(stream)))
+
+    def finalize_device(self, sum_ptr: int, classes_ptr: int, conf_ptr: int, ent_ptr: int, conf32_ptr: int = 0, ent32_ptr: int = 0,
+                        stream: int = 0):
+        """classes / confidence / entropy (+ f32 copies) from the probability sums of all T samples; any output may be 0.
+        The maps become the result semantic_keys reads."""
+        L.check(L.lib().sivo_segnet_finalize_device(self._h, C.c_void_p(sum_ptr), C.c_void_p(classes_ptr), C.c_void_p(conf_ptr),
+                                                    C.c_void_p(ent_ptr), C.c_void_p(conf32_ptr), C.c_void_p(ent32_ptr),
+                                                    C.c_void_p(stream)))
 
     def blob(self, name: str) -> np.ndarray:
         n, c, h, w = C.c_int(), C.c_int(), C.c_int(), C.c_int()
